@@ -20,6 +20,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -40,7 +41,48 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-ops", action="store_true", help="print the per-op breakdown to stderr")
     ap.add_argument("--no-c5", action="store_true", help="skip the BASELINE configs[4] block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
+
+
+DUMP_BUDGET = 64 << 20     # bytes written by --dump-outputs, at most
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir, data, input_keys):
+    """Write what one forward returned to its caller (every key of `data` not in `input_keys`) as
+    out_dir/<name>.npy: float tensors in float32 (float64 stays float64), integer and bool tensors
+    and Python scalars / shapes in float64 (exact).  A tensor of more than 2**20 entries is written
+    as a fixed sample of 2**20 of its flattened entries (seeded by DUMP_SEED, ascending flat indices
+    in <name>_sample_index.npy), halved until all files fit in DUMP_BUDGET.
+    With the same bench arguments the inputs are the same, so the files of two builds compare
+    entry for entry."""
+    arrays = {}
+    for k, v in data.items():
+        if k in input_keys or v is None:
+            continue
+        t = v.detach() if torch.is_tensor(v) else torch.tensor(v, dtype=torch.float64)
+        if t.is_floating_point() and t.dtype != torch.float64:
+            t = t.float()
+        elif not t.is_floating_point():
+            t = t.double()
+        arrays[k] = t
+
+    def nbytes(cap):
+        return sum(min(t.numel(), cap) * t.element_size() + (8 * cap if t.numel() > cap else 0)
+                   for t in arrays.values())
+    cap = 1 << 20
+    while nbytes(cap) > DUMP_BUDGET:
+        cap //= 2
+    os.makedirs(out_dir, exist_ok=True)
+    for k, t in arrays.items():
+        if t.numel() > cap:
+            g = torch.Generator().manual_seed(DUMP_SEED)
+            idx = torch.randint(0, t.numel(), (cap,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+            np.save(os.path.join(out_dir, k + "_sample_index.npy"), idx.double().numpy())
+        np.save(os.path.join(out_dir, k + ".npy"), t.cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------
@@ -175,6 +217,8 @@ def run_reference(args, rank):
     for _ in range(args.steps):
         d = step()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d, set(data))
     val = sample * args.steps / dt
     print(json.dumps({
         "impl": "reference", "metric": "query images/sec (512x512, 5k 3D pts)", "value": val,
@@ -442,6 +486,8 @@ def main():
     _lib.LAUNCHES = 0
     ms, d, t0, t1 = timed(step_resident, args.steps, per_step=True)
     clocks = sampler.stop(t0, t1) if sampler else None
+    if args.dump_outputs and rank == 0:     # before any later forward reuses the workspace
+        dump_outputs(args.dump_outputs, d, set(make_data(imgs_dev, scale_dev, bank)))
     launches = _lib.LAUNCHES
     m_per_img = d["b_ids"].numel() / B
 

@@ -1,5 +1,5 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from /root/reference
-through oracle/ref_shims.py) on small planted workloads — run in the build container only:
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported through
+oracle/ref_shims.py from the checkout at ref_shims.REFERENCE_ROOT) on small planted workloads:
 
     python -m oracle.make_golden
 
@@ -51,7 +51,7 @@ def build_inputs(sd, case):
 
 @torch.no_grad()
 def main():
-    assert ref_shims.available(), "needs /root/reference (build container only)"
+    assert ref_shims.available(), f"no checkout of the original OnePose++ at {ref_shims.REFERENCE_ROOT} (set OPP_REFERENCE_ROOT)"
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     sd = workload.synthetic_state_dict(WEIGHT_SEED)
     model = ref_shims.build_reference_model(sd, oracle.DEFAULT_CONFIG)

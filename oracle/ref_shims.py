@@ -1,5 +1,6 @@
-"""Import the UNMODIFIED reference model from /root/reference in the build container —
-TEST INFRASTRUCTURE ONLY (used to pin oracle/oracle.py and to generate tests/golden/).
+"""Import the UNMODIFIED reference model from a checkout of the original OnePose++ repository
+(REFERENCE_ROOT below; the environment variable OPP_REFERENCE_ROOT points elsewhere) — TEST
+INFRASTRUCTURE ONLY (used to pin oracle/oracle.py and to generate tests/golden/).
 
 The reference needs three packages that are not in this image; each gets a tiny stand-in that
 restates only what the hot path calls (SURVEY.md App. B):
@@ -7,8 +8,8 @@ restates only what the hot path calls (SURVEY.md App. B):
   * kornia.utils.grid.create_meshgrid, kornia.geometry.subpix.dsnt.spatial_expectation2d
     (utils/fine_matching.py:7-8,86-87) — restated from kornia 0.4.1's published definitions
   * src.utils.profiler.PassThroughProfiler (pytorch_lightning dependency)
-/root/reference does not exist on the GPU box: nothing under tests -m gpu, smoke() or bench.py
-may import this module.
+The original sources are not part of this repository: nothing under tests -m gpu, smoke() or
+bench.py may import this module.
 """
 import copy
 import os
@@ -18,7 +19,8 @@ from contextlib import contextmanager
 
 import torch
 
-REFERENCE_ROOT = "/root/reference"
+# where the environment that builds and checks this project keeps the original checkout
+REFERENCE_ROOT = os.environ.get("OPP_REFERENCE_ROOT") or "/root/reference"
 
 
 def available():

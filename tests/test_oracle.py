@@ -1,11 +1,11 @@
-"""CPU tests: the oracle restatement against the committed golden fixtures (generated from the
-unmodified reference, oracle/make_golden.py) and, when /root/reference is present (build
-container), against the reference run live."""
+"""CPU tests: the oracle restatement against the committed golden fixtures generated from the
+unmodified reference (oracle/make_golden.py: stored inputs; oracle/make_reference_runs.py: inputs
+rebuilt from their seeds, the reference's results recorded under tests/golden/reference_runs/)."""
 import numpy as np
 import pytest
 import torch
 
-from oracle import oracle, ref_shims, workload
+from oracle import oracle, workload
 from tests import golden_io
 
 WEIGHTS = {}
@@ -66,42 +66,35 @@ def test_random_workload_has_no_matches():
     assert data["mkpts_query_f"].shape == (0, 2)
 
 
-@pytest.mark.skipif(not ref_shims.available(), reason="/root/reference only exists in the build container")
 @pytest.mark.parametrize("shape", [(96, 128, 300, 120, 2, False, "linear"), (512, 512, 5000, 3000, 1, False, "linear"),
                                    (96, 128, 300, 120, 2, True, "linear"), (96, 128, 300, 120, 2, False, "full")],
                          ids=["small_b2", "baseline_512_n5000", "small_b2_query_mask", "small_b2_full_attention"])
-def test_oracle_matches_reference_live(shape):
+def test_oracle_matches_reference_live(shape, request):
+    """The oracle against the results the unmodified reference computed on the same planted
+    workload (recorded by oracle/make_reference_runs.py)."""
     import copy
+    z = golden_io.reference_run("oracle_" + request.node.callspec.id)
     sd = weights()
     h, w, n, npl, batch, masked, attention = shape
+    assert tuple(z["case"]) == shape[:6] and str(z["attention"]) == attention
     data, meta = workload.planted_workload(sd, h, w, n, npl, batch=batch, seed=5)
     if masked:   # img_pad flow (OnePosePlusModel.py:158): bottom / right of the coarse grid is padding
         data["query_image_mask"] = workload.pad_mask(batch, h // 8, w // 8)
+    golden_io.check_inputs(z, data)
     cfg = copy.deepcopy(oracle.DEFAULT_CONFIG)
     cfg["loftr_coarse"]["attention"] = attention      # "full": FullAttention (linear_attention.py:64-95)
-    if attention == "full":
-        ref = ref_shims.build_reference_model(sd, cfg)
-        d_ref = {k: v.clone() for k, v in data.items()}
-        with torch.no_grad():
-            ref(d_ref)
-        d_or = {k: v.clone() for k, v in data.items()}
-        oracle.forward(sd, d_or, cfg=cfg)
-        # same weights, different attention: the planted bank no longer matches, compare the raw matrix
-        assert torch.allclose(d_ref["conf_matrix"], d_or["conf_matrix"], atol=1e-4)
-        assert torch.equal(d_ref["b_ids"], d_or["b_ids"]) and torch.equal(d_ref["j_ids"], d_or["j_ids"])
-        return
-    ref = ref_shims.build_reference_model(sd, oracle.DEFAULT_CONFIG)
-    d_ref = {k: v.clone() for k, v in data.items()}
-    with torch.no_grad():
-        ref(d_ref)
     d_or = {k: v.clone() for k, v in data.items()}
-    oracle.forward(sd, d_or)
-    assert len(d_ref["b_ids"]) > 20
+    oracle.forward(sd, d_or, cfg=cfg)
+    golden_io.check_conf(z, d_or["conf_matrix"], atol=1e-4)
+    if attention == "full":
+        # same weights, different attention: the planted bank no longer matches, compare the raw matrix
+        assert np.array_equal(z["b_ids"], d_or["b_ids"].numpy()) and np.array_equal(z["j_ids"], d_or["j_ids"].numpy())
+        return
+    assert len(z["b_ids"]) > 20
     for k in ("b_ids", "i_ids", "j_ids", "m_bids", "mkpts_3d_db", "mkpts_query_c"):
-        assert torch.equal(d_ref[k], d_or[k]), k
-    assert torch.allclose(d_ref["conf_matrix"], d_or["conf_matrix"], atol=1e-4)
-    assert torch.allclose(d_ref["mkpts_query_f"], d_or["mkpts_query_f"], atol=2e-3)
-    assert torch.allclose(d_ref["expec_f"][:, :2], d_or["expec_f"][:, :2], atol=2e-4)
+        assert np.array_equal(z[k], d_or[k].numpy()), k
+    assert np.allclose(z["mkpts_query_f"], d_or["mkpts_query_f"].numpy(), atol=2e-3)
+    assert np.allclose(z["expec_f"][:, :2], d_or["expec_f"][:, :2].numpy(), atol=2e-4)
 
 
 def test_pnp_oracle_recovers_planted_poses():
@@ -118,27 +111,28 @@ def test_pnp_oracle_recovers_planted_poses():
         assert np.abs(ref - gt[i]).max() < 5e-3 and np.abs(ref - pose).max() < 2e-3
 
 
-@pytest.mark.skipif(not ref_shims.available(), reason="/root/reference only exists in the build container")
 @pytest.mark.parametrize("case", [(192, 256, 2, False), (256, 320, 1, True)], ids=["b2", "b1_scaled"])
-def test_loftr_oracle_matches_reference_live(case):
-    """oracle/loftr_oracle.py against the unmodified LoFTR_for_OnePose_Plus
-    (src/KeypointFreeSfM/loftr_for_sfm/loftr.py + submodules/LoFTR/src/loftr) on a planted pair."""
+def test_loftr_oracle_matches_reference_live(case, request):
+    """oracle/loftr_oracle.py against the results of the unmodified LoFTR_for_OnePose_Plus
+    (src/KeypointFreeSfM/loftr_for_sfm/loftr.py + submodules/LoFTR/src/loftr) on a planted pair
+    (recorded by oracle/make_reference_runs.py)."""
     from oracle import loftr_oracle
+    z = golden_io.reference_run("loftr_" + request.node.callspec.id)
     h, w, batch, with_scale = case
+    assert tuple(z["case"]) == case
     sd, data = workload.planted_loftr(h, w, batch=batch, with_scale=with_scale)
+    golden_io.check_inputs(z, data)
+    golden_io.check_inputs(z, {k: sd[k] for k in ("loftr_coarse.layers.7.norm2.bias",
+                                                  "backbone.layer1_outconv2.3.weight")}, prefix="sd_")
     cfg = dict(loftr_oracle.DEFAULT_CONFIG)
-    ref = ref_shims.build_reference_loftr(sd, cfg)
-    d_ref = {k: v.clone() for k, v in data.items()}
-    with torch.no_grad():
-        ref(d_ref)
     d_or = loftr_oracle.forward(sd, {k: v.clone() for k, v in data.items()}, cfg)
-    assert len(d_ref["b_ids"]) > 100 * batch
-    off = (d_ref["i_ids"] - d_ref["j_ids"])
-    assert (off == 2 * (w // 8) + 3).float().mean().item() > 0.9      # the planted (16, 24) px shift
+    assert len(z["b_ids"]) > 100 * batch
+    off = (z["i_ids"] - z["j_ids"])
+    assert (off == 2 * (w // 8) + 3).mean() > 0.9      # the planted (16, 24) px shift
     for k in ("b_ids", "i_ids", "j_ids", "mkpts0_c", "mkpts1_c"):
-        assert torch.equal(d_ref[k], d_or[k]), k
-    assert torch.allclose(d_ref["conf_matrix"], d_or["conf_matrix"], atol=1e-4)
-    assert torch.allclose(d_ref["mconf"], d_or["mconf"], atol=1e-4)
-    assert torch.allclose(d_ref["expec_f"][:, :2], d_or["expec_f"][:, :2], atol=2e-4)
-    assert torch.allclose(d_ref["mkpts1_f"], d_or["mkpts1_f"], atol=2e-3) and torch.equal(d_ref["mkpts0_f"], d_or["mkpts0_f"])
-    assert d_ref["W"] == 9
+        assert np.array_equal(z[k], d_or[k].numpy()), k
+    golden_io.check_conf(z, d_or["conf_matrix"], atol=1e-4)
+    assert np.allclose(z["mconf"], d_or["mconf"].numpy(), atol=1e-4)
+    assert np.allclose(z["expec_f"][:, :2], d_or["expec_f"][:, :2].numpy(), atol=2e-4)
+    assert np.allclose(z["mkpts1_f"], d_or["mkpts1_f"].numpy(), atol=2e-3) and np.array_equal(z["mkpts0_f"], d_or["mkpts0_f"].numpy())
+    assert int(z["W"]) == 9
